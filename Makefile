@@ -1,5 +1,6 @@
 # stencil_b200 build: hand-written sm_100a CUDA, no cmake needed.
-#   make            -> stencil_b200/libstencil_b200.so (C ABI + kernels) and lib/libstencil.a (C++ API, -rdc)
+#   make            -> stencil_b200/libstencil_b200.so (C ABI + kernels) and lib/libstencil.a (C++ API, -rdc), plus
+#                      bin/sb_mpirun, bin/jacobi3d_b200 and bin/test_exchange_multigpu (this repository's own drivers)
 #   make drivers    -> bin/ : the REFERENCE's own drivers and Catch2 suites compiled, unchanged, from
 #                      $(REF)/bin and $(REF)/test against OUR headers and library (needs $(REF))
 #   make oracle     -> oracle/_build/liboracle.so (test infrastructure)
@@ -31,7 +32,7 @@ LIBA      := lib/libstencil.a
 # inside libstencil.a would shadow or clash with the real one)
 LIBMPI    := lib/libmpi_shim.a
 
-all: $(SO) $(LIBA) $(LIBMPI) bin/sb_mpirun
+all: $(SO) $(LIBA) $(LIBMPI) bin/sb_mpirun bin/jacobi3d_b200 bin/test_exchange_multigpu
 
 build/mpi_shim.o: src/mpi_shim.cpp include/mpi_shim/mpi.h
 	@mkdir -p build
@@ -67,6 +68,8 @@ $(LIBA): $(APIOBJ) $(CAPIOBJ)
 DRVFLAGS  := -O3 -std=c++14 $(ARCH) -lineinfo -rdc=true --expt-extended-lambda -Xcompiler -w -w -x cu $(APIDEFS) \
              -DCATCH_CONFIG_NO_POSIX_SIGNALS $(APIINC) -I$(REF)/thirdparty -I$(REF)/bin
 DRVLINK    = $(ARCH) -rdc=true -L/usr/local/cuda/lib64/stubs -lnvidia-ml -ldl -lcudart -lrt
+# this repository's own drivers and checks: built by `make` without $(REF)
+OWNFLAGS  := $(filter-out -I$(REF)/thirdparty -I$(REF)/bin,$(DRVFLAGS))
 DRIVERS   := jacobi3d jacobi3d_strong bench_exchange bench_pack exchange_weak exchange_strong
 TESTCUDA  := test_cuda_main test_cuda_align test_cuda_local_domain test_cuda_pack test_cuda_packer test_cuda_rcstream \
              test_cuda_translate test_cuda_translate_kernel test_cuda_gpu_topo test_exchange
@@ -99,7 +102,7 @@ bin/test_cpu: $(patsubst %,build/drv/t_%.o,$(TESTCPU)) $(LIBA)
 # our own driver: the reference's jacobi3d loop over stencil::FusedJacobi3d (no reference sources involved)
 build/drv/jacobi3d_b200.o: drivers/jacobi3d_b200.cu $(wildcard include/stencil/*)
 	@mkdir -p $(dir $@)
-	$(NVCC) $(filter-out -I$(REF)/thirdparty -I$(REF)/bin,$(DRVFLAGS)) -c $< -o $@
+	$(NVCC) $(OWNFLAGS) -c $< -o $@
 bin/jacobi3d_b200: build/drv/jacobi3d_b200.o $(LIBA)
 	@mkdir -p bin
 	$(NVCC) $(DRVLINK) -o $@ $< $(LIBA) $(LIBMPI)
@@ -117,7 +120,10 @@ build/drv/exchange_uniform.o: oracle/ref/ref_exchange_uniform.cu $(wildcard incl
 # our own multi-GPU check of the C++ API
 build/drv/test_exchange_multigpu.o: tests/cpp/test_exchange_multigpu.cu $(wildcard include/stencil/*)
 	@mkdir -p $(dir $@)
-	$(NVCC) $(DRVFLAGS) -c $< -o $@
+	$(NVCC) $(OWNFLAGS) -c $< -o $@
+bin/test_exchange_multigpu: build/drv/test_exchange_multigpu.o $(LIBA) $(LIBMPI)
+	@mkdir -p bin
+	$(NVCC) $(DRVLINK) -o $@ $< $(LIBA) $(LIBMPI)
 
 # the reference's astaroth driver (its own MHD kernels; halos through our library), unchanged
 ASTRO     := astaroth kernels astaroth_utils

@@ -46,7 +46,13 @@ def parse():
                    help="fused: one kernel per iteration = jacobi update + halo push into the neighbours' ghost cells (Jacobi3D.step_fused); "
                    "queued: interior || exchange -> exterior with CUDA-event dependencies (step_async); host-sync: the reference's loop (step)")
     p.add_argument("--host-sync", action="store_true", help="block the host after the exchange and after the exterior kernels like bin/jacobi3d.cu:337-365 (default: iterations queue back to back, dependencies as CUDA events)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the field they computed as DIR/jacobi_field_sample.npy (see dump_outputs)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def measured_peaks():
@@ -308,6 +314,35 @@ def grown_size(n, ngpu, grow):
     return (Z, Y, X) if grow == "cube" else (X, Y, Z)
 
 
+DUMP_POINTS = 1 << 22  # 32 MiB of FP64: the 512^3 field itself is 1 GiB
+DUMP_SEED = 20240517
+
+
+def dump_outputs(out_dir, dd, h, size, dtype, rank, world):
+    """--dump-outputs: the field the timed steps left in curr (what a caller of the jacobi loop reads back), at DUMP_POINTS
+    cells drawn with a fixed seed from the global X x Y x Z domain -- the same cells for every partition, process count and
+    build -- in the run's dtype, as out_dir/jacobi_field_sample.npy on rank 0."""
+    import torch
+    import torch.distributed as td
+
+    X, Y, Z = size
+    rng = np.random.default_rng(DUMP_SEED)
+    pts = np.stack([rng.integers(0, Z, DUMP_POINTS), rng.integers(0, Y, DUMP_POINTS), rng.integers(0, X, DUMP_POINTS)], axis=1)  # z, y, x
+    vals = np.zeros(DUMP_POINTS, dtype=dtype)
+    for d in dd.domains():
+        lo = np.array(d.origin()[::-1])
+        inside = np.all((pts >= lo) & (pts < lo + np.array(d.size()[::-1])), axis=1)
+        q = pts[inside] - lo
+        vals[inside] = d.interior_to_host(h.id)[q[:, 0], q[:, 1], q[:, 2]]
+    if world > 1:
+        t = torch.from_numpy(vals).cuda()
+        td.all_reduce(t)  # every cell lives on one rank; the others add zeros
+        vals = t.cpu().numpy()
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "jacobi_field_sample.npy"), vals)
+
+
 def run_ours(args, rank, world):
     import torch
     import torch.distributed as td
@@ -418,6 +453,8 @@ def run_ours(args, rank, world):
     ms_step = ms_total / args.steps
     cells = X * Y * Z
     value = cells / (ms_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dd, h, (X, Y, Z), dtype, rank, world)
 
     # ---- roofline of the dominant kernel (interior jacobi) ----------------------------------
     peak, peak_src = measured_peaks()

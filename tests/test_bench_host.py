@@ -43,3 +43,39 @@ def test_reference_order_is_the_size_rule_of_the_driver(bench):
     assert tuple(bench.grown_size(512, 2, "yz")) == (512, 512, 1024)
     assert tuple(bench.grown_size(512, 2, "cube")) == (512, 512, 1024)
     assert tuple(bench.grown_size(512, 8, "cube")) == (1024, 1024, 1024)
+
+
+def test_dump_outputs_samples_the_global_field(bench, tmp_path, monkeypatch):
+    """--dump-outputs reads each seeded global cell from the subdomain that owns it, whatever the partition."""
+    import numpy as np
+
+    X, Y, Z = 40, 30, 50
+    field = np.random.default_rng(0).standard_normal((Z, Y, X))
+
+    class Sub:
+        def __init__(self, origin, size):
+            self.o, self.s = origin, size
+
+        def origin(self):
+            return self.o
+
+        def size(self):
+            return self.s
+
+        def interior_to_host(self, q):
+            (x, y, z), (sx, sy, sz) = self.o, self.s
+            return field[z : z + sz, y : y + sy, x : x + sx].copy()
+
+    class Dom:
+        def domains(self):
+            return [Sub((0, 0, 0), (40, 30, 20)), Sub((0, 0, 20), (40, 16, 30)), Sub((0, 16, 20), (40, 14, 30))]
+
+    class Handle:
+        id = 0
+
+    monkeypatch.setattr(bench, "DUMP_POINTS", 5000)
+    bench.dump_outputs(str(tmp_path), Dom(), Handle(), (X, Y, Z), np.float64, 0, 1)
+    got = np.load(tmp_path / "jacobi_field_sample.npy")
+    rng = np.random.default_rng(bench.DUMP_SEED)
+    z, y, x = rng.integers(0, Z, 5000), rng.integers(0, Y, 5000), rng.integers(0, X, 5000)
+    assert got.dtype == np.float64 and np.array_equal(got, field[z, y, x])
