@@ -14,7 +14,9 @@
  * Parity status: the reference holds NO test for these numerics (astaroth/astaroth.cu:538 "TODO"); the pin is
  * tests/golden/astaroth_solve_ref.npz, produced on a B200 by the reference's own solve<> kernels
  * (oracle/ref/ref_astaroth_solve.cu + oracle/ref/make_astaroth_golden.py).  Floating point: compiled with
- * -ffp-contract=off while nvcc contracts a*b+c into FMAs, so agreement is to rounding, not bit-exact.
+ * -ffp-contract=off while nvcc contracts a*b+c into FMAs, so agreement is to rounding, not bit-exact.  The `f80`
+ * instance (long double: 64-bit mantissa on x86-64) is the reference the FP32 and FP64 kernels are bounded against,
+ * a few ulp of the field's magnitude (tests/astaroth_util.py).
  */
 #include <math.h>
 #include <stdint.h>
@@ -256,3 +258,5 @@ enum { LNRHO = 0, UUX, UUY, UUZ, AX, AY, AZ, ENTROPY, NFIELDS };
 
 AC_TEMPLATE(double, f64, exp)
 AC_TEMPLATE(float, f32, expf)
+/* x87 extended precision (64-bit mantissa): the high-precision reference the GPU kernels are bounded against */
+AC_TEMPLATE(long double, f80, expl)

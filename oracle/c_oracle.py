@@ -83,6 +83,7 @@ def lib() -> C.CDLL:
             getattr(L, "so_fill_" + suf).argtypes = [C.c_void_p, Vec, Vec, Vec, ct]
             getattr(L, "so_sqdiff_" + suf).argtypes = [C.c_void_p, C.c_void_p, Vec, Vec, Vec]
             getattr(L, "so_sqdiff_" + suf).restype = C.c_double
+        for suf in ("f32", "f64", "f80"):
             getattr(L, "so_astaroth_substep_" + suf).argtypes = [
                 C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int64, C.c_int64,
                 C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(AcParams),
@@ -152,9 +153,15 @@ def sqdiff(a: np.ndarray, b: np.ndarray, pos, ext) -> float:
     return getattr(lib(), "so_sqdiff_" + _suffix(a))(a.ctypes.data, b.ctypes.data, _raw(a), Vec.of(pos), Vec.of(ext))
 
 
+def longdouble_is_extended() -> bool:
+    """True where np.longdouble is the x87 80-bit format (64-bit mantissa), i.e. the `f80` oracle is a real reference."""
+    return np.finfo(np.longdouble).nmant >= 63
+
+
 def astaroth_substep(step: int, fin, fout, lo, hi, params: "AcParams") -> None:
     """solve<step> on the memory-offset box [lo, hi) (astaroth/kernels.cu:62-87).  fin / fout: 8 arrays
-    (lnrho, uux, uuy, uuz, ax, ay, az, entropy) of identical (mz, my, mx) shape and dtype; fout is updated in place."""
+    (lnrho, uux, uuy, uuz, ax, ay, az, entropy) of identical (mz, my, mx) shape and dtype (float32, float64, or
+    longdouble for the extended-precision reference); fout is updated in place."""
     a0 = fin[0]
     assert len(fin) == 8 and len(fout) == 8
     for a in list(fin) + list(fout):
@@ -163,4 +170,9 @@ def astaroth_substep(step: int, fin, fout, lo, hi, params: "AcParams") -> None:
     pin = (C.c_void_p * 8)(*[a.ctypes.data for a in fin])
     pout = (C.c_void_p * 8)(*[a.ctypes.data for a in fout])
     clo, chi = (C.c_int64 * 3)(*lo), (C.c_int64 * 3)(*hi)
-    getattr(lib(), "so_astaroth_substep_" + _suffix(a0))(step, pin, pout, mx, my, clo, chi, C.byref(params))
+    if a0.dtype == np.longdouble:
+        assert longdouble_is_extended(), "np.longdouble is not the 80-bit format the f80 oracle is compiled for"
+        suf = "f80"
+    else:
+        suf = _suffix(a0)
+    getattr(lib(), "so_astaroth_substep_" + suf)(step, pin, pout, mx, my, clo, chi, C.byref(params))

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import stencil_b200 as sb
-from astaroth_util import GOLDEN, make_fields, tolerance
+from astaroth_util import BOXES, GOLDEN, make_fields, tolerance
 from gpu_util import DevArray
 from oracle import c_oracle as co
 from oracle import geometry as g
@@ -43,18 +43,6 @@ def assert_close(got, want, dtype, what):
         scale = max(1.0, float(np.abs(b).max()))
         err = float(np.abs(a.astype(np.float64) - b.astype(np.float64)).max())
         assert err <= tol * scale, (what, ac.FIELDS[f], err, scale)
-
-
-BOXES = [
-    # raw size (x,y,z), lo, hi
-    ((38, 34, 30), (3, 3, 3), (35, 31, 27)),  # the whole compute region, partial tiles in x and y
-    ((70, 26, 41), (3, 3, 3), (67, 23, 38)),
-    ((40, 40, 40), (6, 6, 6), (34, 34, 34)),  # an interior region
-    ((40, 40, 40), (3, 3, 3), (6, 37, 37)),  # x-face exterior slab (thin -> cell kernel under AUTO)
-    ((40, 40, 40), (6, 34, 3), (34, 37, 37)),  # y-face slab
-    ((40, 40, 40), (6, 6, 34), (34, 34, 37)),  # z-face slab
-    ((23, 22, 21), (5, 4, 3), (16, 17, 18)),
-]
 
 
 @pytest.mark.parametrize("dtype", [np.float64, np.float32])
