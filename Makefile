@@ -11,7 +11,8 @@ NVCCFLAGS := -O3 -std=c++17 $(ARCH) -lineinfo -Xcompiler -fPIC -Xcompiler -Wall 
 INC       := -Iinclude -Istencil_b200/csrc
 
 # ---- core: kernels + C ABI (shared library, loaded by python and linked by the C++ API)
-CSRC      := stencil_b200/csrc/box_copy.cu stencil_b200/csrc/jacobi.cu stencil_b200/csrc/astaroth.cu stencil_b200/csrc/capi.cu
+CSRC      := stencil_b200/csrc/box_copy.cu stencil_b200/csrc/jacobi.cu stencil_b200/csrc/astaroth.cu stencil_b200/csrc/reduce.cu \
+             stencil_b200/csrc/capi.cu
 COBJ      := $(patsubst stencil_b200/csrc/%.cu,build/csrc/%.o,$(CSRC))
 SO        := stencil_b200/libstencil_b200.so
 

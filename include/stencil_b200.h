@@ -217,6 +217,39 @@ int sb_sqdiff(sb_pitched a, sb_pitched b, int dtype_size, const int64_t acc_orig
               const int64_t hi[3], double *out_dev, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Field reductions: the filters of the reference's astaroth extract (astaroth/reductions.cuh:18-52) over a box of
+ * 1-4 operand allocations with the same pitch and ysize.  Per cell a value f and a square g are evaluated in FP64
+ * (FP32 inputs are widened; VALUE, DIFF and VECTOR round every operation, so f is bit-identical to float64 numpy):
+ *   VALUE  (a)          f = a                            g = a*a
+ *   DIFF   (a, b)       f = a - b                        g = (a - b)^2
+ *   VECTOR (a, b, c)    f = sqrt(s), s = (a*a + b*b) + c*c   g = s
+ *   EXP    (a)          f = exp(a)                       g = exp(a)*exp(a)
+ *   ALFVEN (a, b, c, d) f = sqrt(s) / sqrt(4 pi exp(d))  g = s / (4 pi exp(d))
+ * and the launch returns min f, max f, sum f, sum g (FP64 sums).  NaN propagates to all four; an empty box gives
+ * +inf, -inf, 0, 0.  RTYPE_MAX / MIN / SUM are max / min / sum; RTYPE_RMS, RMS_EXP and ALFVEN_RMS are sqrt(sum2 / cells).
+ * Deterministic: no floating-point atomics; the same box on the same GPU gives the same bits on every call.
+ * ------------------------------------------------------------------------------------------- */
+typedef enum sb_reduce_kind {
+  SB_REDUCE_VALUE = 0,
+  SB_REDUCE_DIFF = 1,
+  SB_REDUCE_VECTOR = 2,
+  SB_REDUCE_EXP = 3,
+  SB_REDUCE_ALFVEN = 4
+} sb_reduce_kind;
+typedef struct {
+  double min, max, sum, sum2;
+} sb_reduce_result;
+/* Bytes of device memory one sb_reduce launch on `device` needs as workspace.  The caller zeroes a workspace once;
+ * every launch leaves it ready for the next.  One workspace serves one launch at a time: concurrent reductions (other
+ * streams) need their own. */
+int64_t sb_reduce_workspace_bytes(int device);
+/* One launch on `stream`: reduces [lo, hi) (global coordinates; acc_origin = global coordinate of allocation element
+ * (0,0,0), as in sb_sqdiff) of operands[0 .. n) (n = 1, 2, 3, 1, 4 by kind), and stores an sb_reduce_result at the start
+ * of `workspace` (device memory) when the launch completes. */
+int sb_reduce(int kind, const sb_pitched *operands, int dtype_size, const int64_t acc_origin[3], const int64_t lo[3],
+              const int64_t hi[3], void *workspace, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Device memory + peer plumbing used by the host layers (C++ and Python).
  * ------------------------------------------------------------------------------------------- */
 int sb_device_count(int *count);

@@ -23,5 +23,6 @@ from .domain import (  # noqa: F401
     prime_factors,
     raw_size,
 )
+from .reduce import ALFVEN, DIFF, EXP, VALUE, VECTOR, Stats, Workspace, reduce_box  # noqa: F401
 
 __all__ = [n for n in dir() if not n.startswith("_")]

@@ -59,6 +59,12 @@ class StepSync(C.Structure):
     _fields_ = [("wait_rows", C.c_void_p * 6), ("signal_rows", C.c_void_p * 6), ("wait_value", C.c_uint32), ("signal_value", C.c_uint32)]
 
 
+class ReduceResult(C.Structure):
+    """sb_reduce_result: min f, max f, sum f, sum g of one reduction (see stencil_b200.reduce)."""
+
+    _fields_ = [(n, C.c_double) for n in ("min", "max", "sum", "sum2")]
+
+
 # every symbol include/stencil_b200.h declares: (restype, argtypes)
 _SIGS = {
     "sb_last_error": (C.c_char_p, []),
@@ -92,6 +98,8 @@ _SIGS = {
     "sb_jacobi3d_fused_sync": (C.c_int, [Pitched, Pitched, C.c_int, I3, I3, I3, I3, I3, C.POINTER(HaloPush), C.POINTER(StepSync), C.c_void_p]),
     "sb_fill": (C.c_int, [Pitched, C.c_int, I3, I3, I3, C.c_double, C.c_void_p]),
     "sb_sqdiff": (C.c_int, [Pitched, Pitched, C.c_int, I3, I3, I3, C.c_void_p, C.c_void_p]),
+    "sb_reduce_workspace_bytes": (C.c_int64, [C.c_int]),
+    "sb_reduce": (C.c_int, [C.c_int, C.POINTER(Pitched), C.c_int, I3, I3, I3, C.c_void_p, C.c_void_p]),
     "sb_device_count": (C.c_int, [C.POINTER(C.c_int)]),
     "sb_malloc": (C.c_int, [C.POINTER(C.c_void_p), C.c_size_t, C.c_int]),
     "sb_free": (C.c_int, [C.c_void_p, C.c_int]),

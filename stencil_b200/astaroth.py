@@ -106,6 +106,18 @@ class Astaroth:
         for s in self.streams + self.ext_streams:
             s.synchronize()
 
+    def diagnostics(self) -> dict:
+        """What an astaroth run reports between iterations: {"uu": Stats of the length of (uux, uuy, uuz), and for each of
+        FIELDS: Stats of its values} over the whole distributed compute region (stencil_b200.reduce: min, max, sum, rms).
+        Waits for the solver's queued work first; collective across ranks like DistributedDomain.reduce."""
+        from . import reduce as _r
+
+        self.synchronize()
+        out = {"uu": self.dd.reduce(_r.VECTOR, self.handles[1:4], streams=self.streams)}
+        for name, h in zip(FIELDS, self.handles):
+            out[name] = self.dd.reduce(_r.VALUE, [h], streams=self.streams)
+        return out
+
     def step(self) -> None:
         """One iteration = three substeps + swap, exactly the loop body of astaroth/astaroth.cu:551-640 (the exchange
         of every substep re-sends the same `curr`: the reference never swaps between substeps)."""

@@ -16,6 +16,7 @@
 #include "box_copy.cuh"
 #include "astaroth.cuh"
 #include "jacobi.cuh"
+#include "reduce.cuh"
 
 #include "stencil/geometry.hpp"
 #include "stencil/partition_core.hpp"
@@ -918,6 +919,64 @@ int sb_sqdiff(sb_pitched a, sb_pitched b, int dtype_size, const int64_t acc_orig
   if (b.pitch != a.pitch || b.ysize != a.ysize || !b.ptr || !out_dev) return fail(SB_ERR_INVALID, "mismatched operands");
   g_launches += uint64_t(sb::launch_sqdiff(static_cast<const char *>(a.ptr), static_cast<const char *>(b.ptr), a.pitch,
                                            a.pitch * a.ysize, alo, ahi, dtype_size, out_dev, static_cast<cudaStream_t>(stream)));
+  SB_CUDA(cudaGetLastError());
+  return SB_OK;
+}
+
+// ----------------------------------------------------------------------------------------- reductions
+// SM count of a device (the reduction grid is a fixed multiple of it), cached: it is read on every launch
+static int sm_count(int device, int *out) {
+  static std::atomic<int> cache[64];
+  if (device >= 0 && device < 64 && cache[device].load() > 0) {
+    *out = cache[device].load();
+    return SB_OK;
+  }
+  int n = 0;
+  SB_CUDA(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, device));
+  if (device >= 0 && device < 64) cache[device].store(n);
+  *out = n;
+  return SB_OK;
+}
+
+int64_t sb_reduce_workspace_bytes(int device) {
+  int n = 0;
+  const int rc = sm_count(device, &n);
+  return rc != SB_OK ? int64_t(rc) : sb::reduce_workspace_bytes(n);
+}
+
+int sb_reduce(int kind, const sb_pitched *operands, int dtype_size, const int64_t acc_origin[3], const int64_t lo[3], const int64_t hi[3],
+              void *workspace, void *stream) {
+  const int n = sb::reduce_num_operands(kind);
+  if (n == 0) return fail(SB_ERR_INVALID, "reduction kind %d (0 VALUE, 1 DIFF, 2 VECTOR, 3 EXP, 4 ALFVEN)", kind);
+  if (!operands || !acc_origin || !lo || !hi || !workspace) return fail(SB_ERR_INVALID, "null argument to sb_reduce");
+  if (reinterpret_cast<uintptr_t>(workspace) % 16 != 0) return fail(SB_ERR_INVALID, "workspace must be 16-byte aligned");
+  int alo[3], ahi[3];
+  int rc = to_alloc_box(operands[0], dtype_size, acc_origin, lo, hi, alo, ahi);
+  if (rc != SB_OK) return rc;
+  const char *ops[4] = {nullptr, nullptr, nullptr, nullptr};
+  for (int o = 0; o < n; ++o) {
+    const sb_pitched &p = operands[o];
+    if (!p.ptr) return fail(SB_ERR_INVALID, "operand %d is null", o);
+    if (p.pitch != operands[0].pitch || p.ysize != operands[0].ysize)
+      return fail(SB_ERR_INVALID, "operand %d: pitch/ysize (%lld, %lld) differ from operand 0 (%lld, %lld)", o, (long long)p.pitch,
+                  (long long)p.ysize, (long long)operands[0].pitch, (long long)operands[0].ysize);
+    if (reinterpret_cast<uintptr_t>(p.ptr) % unsigned(dtype_size) != 0) return fail(SB_ERR_INVALID, "operand %d is not aligned to its element size", o);
+    ops[o] = static_cast<const char *>(p.ptr);
+  }
+  if (operands[0].pitch % dtype_size != 0) return fail(SB_ERR_INVALID, "pitch %lld is not a multiple of the element size", (long long)operands[0].pitch);
+  for (int k = 0; k < 3; ++k)
+    if (ahi[k] < alo[k]) return fail(SB_ERR_INVALID, "box has hi < lo on axis %d", k);
+  const bool empty = ahi[0] == alo[0] || ahi[1] == alo[1] || ahi[2] == alo[2];
+  if (!empty && ahi[0] > operands[0].pitch / dtype_size) return fail(SB_ERR_INVALID, "box ends at x = %d, past the row of %lld elements", ahi[0], (long long)(operands[0].pitch / dtype_size));
+  if (!empty && ahi[1] > operands[0].ysize) return fail(SB_ERR_INVALID, "box ends at y = %d, past the %lld rows of a plane", ahi[1], (long long)operands[0].ysize);
+  if (int64_t(ahi[1] - alo[1]) * int64_t(ahi[2] - alo[2]) >= (1ll << 31)) return fail(SB_ERR_INVALID, "box has 2^31 rows or more");
+  PtrDeviceGuard guard(operands[0].ptr);
+  int dev = 0, sms = 0;
+  SB_CUDA(cudaGetDevice(&dev));
+  rc = sm_count(dev, &sms);
+  if (rc != SB_OK) return rc;
+  g_launches += uint64_t(sb::launch_reduce(kind, ops, dtype_size, operands[0].pitch, operands[0].pitch * operands[0].ysize, alo, ahi, workspace,
+                                           sms, static_cast<cudaStream_t>(stream)));
   SB_CUDA(cudaGetLastError());
   return SB_OK;
 }

@@ -401,6 +401,7 @@ class DistributedDomain:
         self._nccl = None  # NCCL fallback (dist.NcclExchange)
         self._use_nccl = False
         self._epoch = 0
+        self._reduce_ws = {}  # local subdomain -> reduce.Workspace, allocated by the first reduce()
 
     # -- configuration (call before realize)
     def set_radius(self, r) -> None:
@@ -751,7 +752,39 @@ class DistributedDomain:
             d.swap()
         self._parity ^= 1
 
+    def reduce(self, kind: int, handles, which: str = "curr", streams=None):
+        """Reduction of `kind` (stencil_b200.reduce: VALUE, DIFF, VECTOR, EXP, ALFVEN) over the whole compute region ->
+        reduce.Stats.  `handles` are the operands in order, each a DataHandle (read from `which` buffer) or a
+        (DataHandle, "curr" | "next") pair; they must share one dtype.  One launch per local subdomain on streams[i] (default:
+        each GPU's current torch stream), waited for here.  Collective like exchange(): every rank must call it, and every
+        rank gets the same bits -- the per-subdomain results are combined in global subdomain index order, so the result
+        also does not depend on how the subdomains are spread over ranks and GPUs."""
+        from . import reduce as _r
+
+        ops = [(h, which) if isinstance(h, DataHandle) else (h[0], h[1]) for h in handles]
+        if len({np.dtype(self.dtypes_[h.id]) for h, _ in ops}) > 1:
+            raise _lib.StencilError("reduction operands must have the same dtype")
+        if any(w not in ("curr", "next") for _, w in ops):
+            raise ValueError("which must be 'curr' or 'next'")
+        if streams is None:
+            import torch
+
+            streams = [torch.cuda.current_stream(d.gpu()) for d in self.domains_]
+        for di, (d, s) in enumerate(zip(self.domains_, streams)):
+            if di not in self._reduce_ws:
+                self._reduce_ws[di] = _r.Workspace(d.gpu())
+            lo, hi = d.get_compute_region()
+            self._reduce_ws[di].launch(kind, [d.pitched(h.id, w) for h, w in ops], d.elem_size(ops[0][0].id), d.accessor_origin(), lo, hi, s)
+        local = {}
+        for di, (d, s) in enumerate(zip(self.domains_, streams)):
+            lo, hi = d.get_compute_region()
+            local[tuple(self.domain_idx_[di])] = self._reduce_ws[di].result(s) + (_r.cells(lo, hi),)
+        return _r.combine_ranks(local, self.partition_.indices(), self._world.size)
+
     def close(self) -> None:
+        for ws in self._reduce_ws.values():
+            ws.free()
+        self._reduce_ws = {}
         for plans in self._plans + getattr(self, "_unpack_plans", []):
             for p in plans:
                 if p is not None:

@@ -9,6 +9,7 @@ handful of foreign calls.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Tuple
 
 import numpy as np
@@ -561,6 +562,15 @@ class Jacobi3D:
         if self.overlap:
             for s in self.ext_streams:
                 s.synchronize()
+
+    def residual(self) -> float:
+        """||curr - next||_2 over the whole distributed compute region: after a step, the change of the last iteration
+        (u_{n+1} - u_n), accumulated in FP64.  Waits for the queued iterations; collective across ranks."""
+        from . import reduce as _r
+
+        self.synchronize()
+        h = self.h
+        return math.sqrt(self.dd.reduce(_r.DIFF, [(h, "curr"), (h, "next")], streams=self.streams).sum2)
 
     def init(self, value: float = 0.5) -> None:
         """init_kernel (bin/jacobi3d.cu:18-29) on curr; ghost cells are filled by the first exchange."""
